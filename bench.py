@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- KV-cache transfer GB/s (+ decode TTFT delta) for the prefill->decode hand-off.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload = BASELINE.json configs[1]: Llama-3-8B bf16, 4 k-token context, paged KV block_size=16
@@ -46,6 +46,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -301,6 +302,24 @@ def verify_destination(torch, dst_bufs, dev, sid, did, cast, lut=None, src_regio
 def golden_lut(torch, dev):
     t = np.load(os.path.join(ROOT, "tests", "golden", "fp8_e4m3_to_bf16_torch.npy"))
     return torch.as_tensor(t.astype(np.uint16).view(np.int16).copy(), device=dev)
+
+
+DUMP_SAMPLES = 4 << 20   # bytes sampled over all destinations: 16 MiB of float32 per run
+
+
+def dump_destination(torch, out_dir, name, dst_bufs, dev, did, n_samples):
+    """Writes out_dir/<name>.npy: a fixed, seeded sample of the bytes this destination received, read the way its owner
+    reads them (layer, K/V, position in the block table, byte), each byte as a float32 in 0..255."""
+    per_layer = OUTER * N_BLOCKS * REGION
+    idx = np.sort(np.random.default_rng(7).integers(0, NL * per_layer, n_samples, dtype=np.int64))
+    layer, rest = np.divmod(idx, per_layer)
+    outer, rest = np.divmod(rest, N_BLOCKS * REGION)
+    j, byte = np.divmod(rest, REGION)
+    offset = torch.as_tensor(outer * (POOL_BLOCKS * REGION) + np.asarray(did, dtype=np.int64)[j] * REGION + byte, device=dev)
+    bounds = np.searchsorted(layer, np.arange(NL + 1))
+    got = torch.cat([dst_bufs[l][offset[bounds[l]:bounds[l + 1]]] for l in range(NL)])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), got.float().cpu().numpy())
 
 
 # =====================================================================================================
@@ -574,6 +593,9 @@ def run_ours(args):
               "how": "device-side comparison of every moved (block, layer, K/V) region with the closed-form source pattern"
                      + (" through the golden fp8->bf16 table (tests/golden)" if CAST else "") + "; every non-destination block must still be zero"}
     ok = parity["ok"]
+    if args.dump_outputs and is_dst:
+        dump_destination(torch, args.dump_outputs, f"received_kv_rank{rank}", dst_bufs, dev, dids[my_dst_index],
+                         DUMP_SAMPLES // (n_dst * n_src))
 
     # ================= extras (not timed): sorted tables, GPU baselines, the other transfer modes =================
     extras = {}
@@ -962,7 +984,12 @@ def main():
                     help="N > 1: pull = every decode GPU launches and reads the prefill pool (default); push = the prefill GPU stores to all")
     ap.add_argument("--topology", default="fanout", choices=["fanout", "pairs"],
                     help="fanout: rank 0 -> ranks 1..N-1 (default); pairs: rank r -> rank r+N/2 (TP-sharded prefill -> decode)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write a seeded sample of the KV bytes every destination received to "
+                         "DIR/received_kv_rank<r>.npy (float32, 16 MiB in all; identical inputs on every run)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs samples the GPU transfer (--impl ours)")
     configure(args)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":

@@ -1,7 +1,8 @@
 /* A C program built against the SIX reference symbols only (lib/kvbm-kernels/src/tensor_kernels.rs:46-109).  The test
- * runs the same binary twice -- LD_LIBRARY_PATH pointing at this repo's libkvbm_kernels.so, then at the reference's own
- * kernels compiled unmodified (oracle/_ref) under the same file name -- and requires byte-identical output: the
- * "swap the .so" drop-in of INTEGRATION.md section 1, literally.  Prints a checksum line per case. */
+ * runs it with LD_LIBRARY_PATH pointing at this repo's libkvbm_kernels.so and requires byte-identical output to what the
+ * same binary printed on the reference's own kernels compiled unmodified (oracle/_ref) under the same file name
+ * (tests/golden/reference_kernels_dropin.txt): the "swap the .so" drop-in of INTEGRATION.md section 1, literally.
+ * Prints a checksum line per case. */
 #include <cuda_runtime_api.h>
 #include <stdint.h>
 #include <stdio.h>

@@ -4,10 +4,11 @@ Mirrors the reference's kernel tests:
   lib/kvbm-kernels/tests/memcpy_batch.rs       (no-ops, H2D+D2H roundtrips over all 3 modes, KAT patterns)
   lib/kvbm-kernels/tests/kernel_roundtrip.rs   (permute roundtrip x dtype x layout, poison fill, empty batch)
   lib/kvbm-kernels/src/tensor_kernels.rs:286-  (universal_roundtrip with +0.25 encoded values)
-and compares every result bit-for-bit with the CPU oracle, and with the reference's own kernels
-(oracle/_ref/libkvbm_kernels_ref.so, compiled unmodified) when that library is present.
+and compares every result bit-for-bit with the CPU oracle, and with what the reference's own kernels
+(tensor_kernels.cu compiled unmodified for sm_100) produced on a B200 for the same inputs, stored under
+tests/golden/ by tests/golden/make_reference_goldens.py.
 """
-import ctypes as C
+import hashlib
 import os
 
 import numpy as np
@@ -21,18 +22,51 @@ from tests.gpu_util import dev_ptr_table, dev_u8, pinned_u8, stream_ptr
 
 pytestmark = pytest.mark.gpu
 
-REF_SO = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref",
-                      "libkvbm_kernels_ref.so")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+REF_COPY_SHA256 = os.path.join(GOLDEN, "reference_vectorized_copy_sha256.npy")
+REF_POSITION_BLOCKS = os.path.join(GOLDEN, "reference_block_from_universal_position_encoded.npy")
 
 
-def ref_lib():
-    if not os.path.exists(REF_SO):
-        return None
-    L = C.CDLL(REF_SO)
-    L.kvbm_kernels_launch_vectorized_copy.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]
-    for f in (L.kvbm_kernels_launch_universal_from_block, L.kvbm_kernels_launch_block_from_universal):
-        f.argtypes = [C.c_void_p, C.c_void_p] + [C.c_size_t] * 6 + [C.c_int, C.c_int, C.c_void_p]
-    return L
+def reference_copy_case():
+    """512 pairs of one 32 KiB (block, layer, outer) region of Llama-3-8B bf16, gathered from a 1024-region pool and
+    scattered in a shuffled order.  Seeded: the reference kernel's output for exactly these inputs is stored."""
+    size, pairs = 32768, 512
+    rng = np.random.default_rng(139)
+    pool = rng.integers(0, 256, (pairs * 2, size), dtype=np.uint8)
+    return size, pairs, pool, rng.permutation(pairs * 2)[:pairs], rng.permutation(pairs)
+
+
+def launch_reference_copy_case(launch):
+    """Runs `launch` (a kvbm_kernels_launch_vectorized_copy) on reference_copy_case(); returns (output, pool, perm, dperm)
+    on the device, output[dperm[i]] being the copy of pool[perm[i]]."""
+    size, pairs, pool, perm, dperm = reference_copy_case()
+    pool = torch.from_numpy(pool).cuda()
+    out = dev_u8(pairs * size).view(pairs, size)
+    st = dev_ptr_table([pool[int(i)].data_ptr() for i in perm])
+    dt = dev_ptr_table([out[int(i)].data_ptr() for i in dperm])
+    assert launch(st.data_ptr(), dt.data_ptr(), size, pairs, stream_ptr()) == 0
+    torch.cuda.synchronize()
+    return out, pool, torch.from_numpy(perm).cuda(), torch.from_numpy(dperm).cuda()
+
+
+def row_sha256(rows: np.ndarray) -> np.ndarray:
+    return np.stack([np.frombuffer(hashlib.sha256(r.tobytes()).digest(), dtype=np.uint8) for r in rows])
+
+
+def block_from_universal_position_encoded(launch_block_from_universal, layout):
+    """The position-encoded universal tensor of kernel_roundtrip.rs:418-493 scattered into its nl*no chunks by the given
+    kvbm_kernels_launch_block_from_universal; returns the chunks as float32 arrays."""
+    d = kats.PERMUTE_DIMS
+    uni = kats.position_encoded_universal(**d)
+    du = torch.from_numpy(uni.reshape(-1).view(np.uint8).copy()).cuda()
+    ut = dev_ptr_table([du.data_ptr()])
+    chunks = [dev_u8(w.nbytes, fill=0xDE) for w in kats.make_blocks(uni, layout)]
+    bt = dev_ptr_table([t.data_ptr() for t in chunks])
+    rc = launch_block_from_universal(ut.data_ptr(), bt.data_ptr(), 1, d["nh"], d["nl"], d["no"], d["nt"], d["hd"], 2, layout,
+                                     stream_ptr())
+    assert rc == 0
+    torch.cuda.synchronize()
+    return [c.cpu().numpy().view(np.float32) for c in chunks]
 
 
 def test_not_a_stub_and_batch_query():
@@ -137,21 +171,9 @@ def test_vectorized_copy_one_huge_pair_is_split_over_the_chip():
 
 
 def test_vectorized_copy_matches_reference_kernel_bit_for_bit():
-    R = ref_lib()
-    if R is None:
-        pytest.skip("oracle/_ref not built")
-    size, pairs = 32768, 512   # one (block,layer,outer) region of Llama-3-8B bf16 per pair
-    pool = torch.randint(0, 256, (pairs * 2, size), dtype=torch.uint8, device="cuda")
-    perm = torch.randperm(pairs * 2)[:pairs]
-    ours, theirs = dev_u8(pairs * size).view(pairs, size), dev_u8(pairs * size).view(pairs, size)
-    dperm = torch.randperm(pairs)
-    st = dev_ptr_table([pool[int(i)].data_ptr() for i in perm])
-    d1 = dev_ptr_table([ours[int(i)].data_ptr() for i in dperm])
-    d2 = dev_ptr_table([theirs[int(i)].data_ptr() for i in dperm])
-    assert K.vectorized_copy(st.data_ptr(), d1.data_ptr(), size, pairs, stream_ptr()) == 0
-    assert R.kvbm_kernels_launch_vectorized_copy(st.data_ptr(), d2.data_ptr(), size, pairs, stream_ptr()) == 0
-    torch.cuda.synchronize()
-    assert torch.equal(ours, theirs)
+    ours, pool, perm, dperm = launch_reference_copy_case(K.vectorized_copy)
+    theirs = np.load(REF_COPY_SHA256)          # SHA-256 of every output row the reference kernel wrote
+    assert np.array_equal(row_sha256(ours.cpu().numpy()), theirs)
     assert torch.equal(ours[dperm], pool[perm])
 
 
@@ -204,28 +226,12 @@ def test_permute_llama70b_tp_reshard_shape(layout):
 
 @pytest.mark.parametrize("layout", [kats.NHD, kats.HND])
 def test_permute_position_encoded_kat_and_reference_kernel(layout):
-    d = kats.PERMUTE_DIMS
-    dims = (d["nh"], d["nl"], d["no"], d["nt"], d["hd"])
-    uni = kats.position_encoded_universal(**d)
-    want = kats.make_blocks(uni, layout)
-    sp = stream_ptr()
-    du = torch.from_numpy(uni.reshape(-1).view(np.uint8).copy()).cuda()
-    ut = dev_ptr_table([du.data_ptr()])
-    outs = {}
-    for name, L in (("ours", K.lib()), ("ref", ref_lib())):
-        if L is None:
-            continue
-        chunks = [dev_u8(w.nbytes, fill=0xDE) for w in want]
-        bt = dev_ptr_table([t.data_ptr() for t in chunks])
-        rc = L.kvbm_kernels_launch_block_from_universal(ut.data_ptr(), bt.data_ptr(), 1, *dims, 2, layout, sp)
-        assert rc == 0
-        torch.cuda.synchronize()
-        outs[name] = [c.cpu().numpy().view(np.float32) for c in chunks]
-    for got, w in zip(outs["ours"], want):
+    ours = block_from_universal_position_encoded(K.lib().kvbm_kernels_launch_block_from_universal, layout)
+    want = kats.make_blocks(kats.position_encoded_universal(**kats.PERMUTE_DIMS), layout)
+    for got, w in zip(ours, want):
         assert np.array_equal(got, w)
-    if "ref" in outs:
-        for a, b in zip(outs["ours"], outs["ref"]):
-            assert np.array_equal(a, b)
+    theirs = np.load(REF_POSITION_BLOCKS)[layout]   # [nl*no, chunk] float32 the reference kernel wrote, per layout
+    assert np.array_equal(np.stack(ours), theirs)
 
 
 def test_universal_roundtrip_quarter_offsets():

@@ -262,7 +262,7 @@ __global__ void __launch_bounds__(512, 1) ws_engine_kernel(const __grid_constant
   ss.ctl = ctl;
   ss.total_rings = gridDim.x * (blockDim.x >> 6);
   ss.layer_end = 1;
-  RingParams rp{S, P, B, gen.j.tile, 0, true, false, 0, 0};
+  RingParams rp{S, P, B, gen.j.tile, 0, true, false, false};
   run_rings<0, true>(smem, gen, gen.j.total, 1, rp, ss);
 }
 

@@ -1,7 +1,7 @@
 """Launches ONE variant of the config-2 same-GPU transfer a few times (for ncu captures).
 
     ncu --set full -k regex:kvbm -c 2 python benchmarks/profile_one.py --which ours
-    which: ours | ours:<warps>,<stages>,<tile>[,<pending>[,<ctas>[,<variant>]]] | simt | k1 | ref | torch
+    which: ours | ours:<warps>,<stages>,<tile>[,<pending>[,<ctas>]] | simt | k1 | ref | torch
 """
 import argparse
 import ctypes as C
@@ -52,7 +52,7 @@ for _ in range(a.iters):
         opts = K.PagedCopyOpts()
         if ":" in w:
             v = [int(x) for x in w.split(":")[1].split(",")]
-            opts = K.PagedCopyOpts(warps_per_cta=v[0], stages=v[1], tile_bytes=v[2], stores_in_flight=v[3] if len(v) > 3 else 0, max_ctas=v[4] if len(v) > 4 else 0, variant=v[5] if len(v) > 5 else 0)
+            opts = K.PagedCopyOpts(warps_per_cta=v[0], stages=v[1], tile_bytes=v[2], stores_in_flight=v[3] if len(v) > 3 else 0, max_ctas=v[4] if len(v) > 4 else 0)
         K.check(K.paged_copy(src, [d], n, 0, nl, 0, opts, sp))
     elif w == "simt":
         K.check(K.paged_copy(src, [d], n, 0, nl, 0, K.PagedCopyOpts(force_simt=1), sp))

@@ -46,7 +46,7 @@ def main():
     ap.add_argument("--out", default="gpurun_out/sweep.json")
     ap.add_argument("--peer", action="store_true", help="destination pool on cuda:1 (NVLink peer stores)")
     ap.add_argument("--pull", action="store_true", help="with --peer: SOURCE pool on cuda:1, kernel on cuda:0 reads over NVLink")
-    ap.add_argument("--fine", action="store_true", help="second-round sweep: CTA count x ring shape x L2 hints")
+    ap.add_argument("--fine", action="store_true", help="second-round sweep: CTA count x ring shape")
     a = ap.parse_args()
     torch.cuda.set_device(0)
     ddev = "cuda:0"
@@ -81,40 +81,29 @@ def main():
     results.append(dict(name="torch.copy_", ms=med, gbs_rw=2 * bytes_moved / med / 1e6))
     print(results[-1], flush=True)
 
-    cfgs = [  # (warps, stages, pending stores, tile, ctas, cache_hint, variant)
-        (4, 3, 1, 16384, 0, 0, 0), (2, 3, 1, 32768, 0, 0, 0), (8, 3, 1, 8192, 0, 0, 0), (4, 6, 3, 8192, 0, 0, 0),
-        (6, 2, 1, 16384, 0, 0, 0), (3, 2, 1, 32768, 0, 0, 0), (12, 2, 1, 8192, 0, 0, 0), (16, 3, 1, 4096, 0, 0, 0),
-        # TMA load + SIMT store from smem (slot is free as soon as the warp has stored it)
-        (4, 3, 1, 16384, 0, 0, 1), (8, 3, 1, 8192, 0, 0, 1), (8, 6, 1, 4096, 0, 0, 1), (16, 3, 1, 4096, 0, 0, 1),
-        (16, 6, 1, 2048, 0, 0, 1), (12, 4, 1, 4096, 0, 0, 1), (8, 2, 1, 8192, 0, 0, 1), (16, 2, 1, 4096, 0, 0, 1),
-        # diagnostics: loads only / stores only (half the traffic; GB/s printed as if both directions moved)
-        (4, 3, 1, 16384, 0, 0, 2), (4, 6, 1, 8192, 0, 0, 2), (8, 3, 1, 8192, 0, 0, 2), (2, 3, 1, 32768, 0, 0, 2),
-        (4, 3, 1, 16384, 0, 0, 3), (4, 3, 2, 16384, 0, 0, 3), (4, 6, 3, 8192, 0, 0, 3), (4, 6, 5, 8192, 0, 0, 3), (8, 3, 2, 8192, 0, 0, 3),
-        (4, 3, 1, 16384, 74, 0, 0), (4, 3, 1, 16384, 32, 0, 0), (4, 3, 1, 16384, 16, 0, 0), (8, 3, 1, 8192, 16, 0, 1),
+    cfgs = [  # (warps, stages, pending stores, tile, ctas)
+        (4, 3, 1, 16384, 0), (2, 3, 1, 32768, 0), (8, 3, 1, 8192, 0), (4, 6, 3, 8192, 0),
+        (6, 2, 1, 16384, 0), (3, 2, 1, 32768, 0), (12, 2, 1, 8192, 0), (16, 3, 1, 4096, 0),
+        (4, 3, 1, 16384, 74), (4, 3, 1, 16384, 32), (4, 3, 1, 16384, 16),
     ]
     if a.fine:
         cfgs = []
         for shape in [(4, 3, 1, 16384), (4, 6, 3, 8192), (2, 3, 1, 32768), (8, 3, 1, 8192), (2, 6, 3, 16384), (4, 4, 2, 8192)]:
             for ctas in (64, 74, 96, 111, 128, 148):
-                cfgs.append((*shape, ctas, 0, 0))
-        for hint in (1, 2, 3):
-            cfgs += [(4, 3, 1, 16384, 74, hint, 0), (4, 3, 1, 16384, 148, hint, 0), (2, 3, 1, 32768, 74, hint, 0)]
+                cfgs.append((*shape, ctas))
     if a.peer:   # NVLink-bound: how few SMs saturate the link, and how many stores must be in flight
-        cfgs = [(4, 3, 1, 16384, 0, 0, 0), (4, 6, 3, 8192, 0, 0, 0), (4, 6, 5, 8192, 0, 0, 0), (2, 6, 4, 16384, 0, 0, 0),
-                (4, 3, 1, 16384, 0, 0, 1), (8, 3, 1, 8192, 0, 0, 1),
-                (4, 3, 1, 16384, 74, 0, 0), (4, 3, 1, 16384, 32, 0, 0), (4, 3, 1, 16384, 16, 0, 0), (4, 3, 1, 16384, 8, 0, 0),
-                (4, 6, 4, 8192, 32, 0, 0), (4, 6, 4, 8192, 16, 0, 0), (4, 6, 4, 8192, 8, 0, 0), (2, 6, 4, 16384, 16, 0, 0),
-                (2, 6, 4, 16384, 8, 0, 0), (4, 12, 10, 4096, 16, 0, 0), (8, 3, 1, 8192, 16, 0, 1), (8, 3, 1, 8192, 32, 0, 1),
-                (4, 3, 2, 16384, 16, 0, 0), (1, 6, 4, 32768, 16, 0, 0), (1, 6, 4, 32768, 32, 0, 0)]
-    for warps, stages, pend, tile, ctas, hint, variant in cfgs:
-        opts = K.PagedCopyOpts(warps_per_cta=warps, stages=stages, tile_bytes=tile, max_ctas=ctas, stores_in_flight=pend,
-                               cache_hint=hint, variant=variant)
+        cfgs = [(4, 3, 1, 16384, 0), (4, 6, 3, 8192, 0), (4, 6, 5, 8192, 0), (2, 6, 4, 16384, 0),
+                (4, 3, 1, 16384, 74), (4, 3, 1, 16384, 32), (4, 3, 1, 16384, 16), (4, 3, 1, 16384, 8),
+                (4, 6, 4, 8192, 32), (4, 6, 4, 8192, 16), (4, 6, 4, 8192, 8), (2, 6, 4, 16384, 16),
+                (2, 6, 4, 16384, 8), (4, 12, 10, 4096, 16), (4, 3, 2, 16384, 16), (1, 6, 4, 32768, 16), (1, 6, 4, 32768, 32)]
+    for warps, stages, pend, tile, ctas in cfgs:
+        opts = K.PagedCopyOpts(warps_per_cta=warps, stages=stages, tile_bytes=tile, max_ctas=ctas, stores_in_flight=pend)
         rc = K.paged_copy(src, [d], n, 0, nl, 0, opts, sp)
         if rc != 0:
             print("rc", rc, warps, stages, tile)
             continue
         med, best = timed(lambda: K.paged_copy(src, [d], n, 0, nl, 0, opts, sp), flush=flush)
-        results.append(dict(name="paged_tma", warps=warps, stages=stages, pending=pend, tile=tile, ctas=ctas, hint=hint, variant=variant,
+        results.append(dict(name="paged_tma", warps=warps, stages=stages, pending=pend, tile=tile, ctas=ctas,
                             ms=med, ms_min=best, gbs_rw=2 * bytes_moved / med / 1e6))
         print(results[-1], flush=True)
     opts = K.PagedCopyOpts(force_simt=1)

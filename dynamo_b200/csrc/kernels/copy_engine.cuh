@@ -120,9 +120,8 @@ struct RingParams {
   uint32_t tile_out;  // cast rings: bytes per output buffer (2 of them)
   bool allow_tma;
   bool static_schedule;  // diagnostics: round-robin batches even when control words exist
-  int cache_hint;     // bit0 evict_first loads, bit1 evict_first stores
-  int variant;        // 0 = TMA load + TMA store; 1 = TMA load + SIMT store from smem; 4 = TMA load + multimem.st (NVLS);
-                      // 2 = loads only (diagnostic), 3 = stores only (diagnostic)
+  bool multimem;      // TMA load + multimem.st from smem to an NVLS multicast address (byte copies only);
+                      // otherwise TMA load + TMA store
 };
 
 // Per-slot control block the producer fills before it arms the slot's `full` barrier.
@@ -212,19 +211,7 @@ __device__ __forceinline__ void arrive_transfer(const StreamSync& ss)
   if (ss.completion_flag != nullptr) ptx::st_relaxed_sys(ss.completion_flag, aborted ? 0xFFFFFFFFu : ss.completion_value);
 }
 
-// smem -> global by the whole warp (variant 1): 16 B per lane
-__device__ __forceinline__ void warp_store_from_smem(uint8_t* dst, uint32_t src_smem, uint32_t bytes, int lane)
-{
-  uint4* d = reinterpret_cast<uint4*>(dst);
-  const uint32_t n = bytes >> 4;
-  for (uint32_t i = lane; i < n; i += 32) {
-    uint4 v;
-    asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(src_smem + i * 16));
-    ptx::st_stream_v4(d + i, v);
-  }
-}
-
-// smem -> NVLink multicast address (variant 4): one store, the switch delivers it to every bound device
+// smem -> NVLink multicast address (multimem rings): one store, the switch delivers it to every bound device
 __device__ __forceinline__ void warp_store_from_smem_mc(uint8_t* dst, uint32_t src_smem, uint32_t bytes, int lane)
 {
   uint4* d = reinterpret_cast<uint4*>(dst);
@@ -261,8 +248,8 @@ __device__ __forceinline__ void warp_cast_simt(uint8_t* dst, const uint8_t* src,
 // on the ramp), later tickets come from ss.ctl[2] and shrink towards the end of the transfer (guided self-scheduling)
 // so that all rings run dry together.  Without control words the schedule is a static round-robin of batches.
 // ------------------------------------------------------------------------------------------
-// FAST = the plain hot path, known at compile time: one destination, TMA load + TMA store, no cache hints, no gating and
-// no per-layer flags.  A ring is ONE instruction stream per direction, so every instruction of the per-item chain costs
+// FAST = the plain hot path, known at compile time: one destination, TMA load + TMA store, no gating and no per-layer
+// flags.  A ring is ONE instruction stream per direction, so every instruction of the per-item chain costs
 // its full latency (~10 ns); folding the run-time generality away is worth 10 % on the HBM-bound copy
 // (profiles/r02_copylab_libsweep.jsonl vs r02_copylab_engine.jsonl).
 template <int CAST, bool FAST, class Gen>
@@ -271,13 +258,10 @@ __device__ __forceinline__ void ring_producer(const Gen& gen, uint32_t total, ui
 {
   const int lane = threadIdx.x & 31;
   const int ndst = FAST ? 1 : ndst_rt;
-  const int variant = FAST ? 0 : rp.variant;
-  const int cache_hint = FAST ? 0 : rp.cache_hint;
   const bool allow_tma = FAST ? true : rp.allow_tma;
   const bool gate = FAST ? false : ss.gate;
   const int S = rp.S;
   const uint32_t B = static_cast<uint32_t>(rp.batch);
-  const uint64_t policy = cache_hint ? ptx::policy_evict_first() : 0;
   const bool dynamic = ss.ctl != nullptr && !rp.static_schedule;
   int ready_layer = gate ? ss.layer_begin - 1 : 0x7fffffff;
   uint32_t k = 0;          // tickets taken
@@ -345,13 +329,9 @@ __device__ __forceinline__ void ring_producer(const Gen& gen, uint32_t total, ui
         c.layer = static_cast<uint32_t>(layer_i);
         c.bytes = meta_i;
         const uint32_t bytes_i = meta_i & ~kSlotTma;
-        const bool load = (meta_i & kSlotTma) != 0 && variant != 3;
-        if (load) {
+        if (meta_i & kSlotTma) {
           ptx::mbar_arrive_expect_tx(sm.full0 + 8 * slot, bytes_i);
-          if (cache_hint & 1)
-            ptx::bulk_g2s_hint(sm.in0 + slot * rp.tile_in, reinterpret_cast<const void*>(src_i), bytes_i, sm.full0 + 8 * slot, policy);
-          else
-            ptx::bulk_g2s(sm.in0 + slot * rp.tile_in, reinterpret_cast<const void*>(src_i), bytes_i, sm.full0 + 8 * slot);
+          ptx::bulk_g2s(sm.in0 + slot * rp.tile_in, reinterpret_cast<const void*>(src_i), bytes_i, sm.full0 + 8 * slot);
         } else {
           ptx::mbar_arrive(sm.full0 + 8 * slot);
         }
@@ -383,13 +363,11 @@ __device__ __forceinline__ void ring_consumer(const RingSmem& sm, int ndst_rt, c
 {
   const int lane = threadIdx.x & 31;
   const int ndst = FAST ? 1 : ndst_rt;
-  const int variant = FAST ? 0 : rp.variant;
-  const int cache_hint = FAST ? 0 : rp.cache_hint;
+  const bool multimem = FAST ? false : rp.multimem;
   const bool want_layers = FAST ? false : ss.want_layers;
   const int S = rp.S;
   const int P = rp.P;
-  const uint64_t policy = cache_hint ? ptx::policy_evict_first() : 0;
-  const bool deferred_release = CAST == 0 && variant == 0;  // TMA stores read the input slot asynchronously
+  const bool deferred_release = CAST == 0 && !multimem;  // TMA stores read the input slot asynchronously
   uint32_t deferred = 0;  // bit (q & 31): item q's slot is handed back once its bulk store has read it
   int cur_layer = -1;
   uint32_t unpublished = 0;
@@ -448,7 +426,7 @@ __device__ __forceinline__ void ring_consumer(const RingSmem& sm, int ndst_rt, c
       const uint8_t* src = reinterpret_cast<const uint8_t*>(c.src);
       for (int d = 0; d < ndst; ++d) {
         uint8_t* dst = reinterpret_cast<uint8_t*>(c.dst[d]);
-        if (CAST == 0 && variant == 4)
+        if (CAST == 0 && multimem)
           warp_copy_simt_mc(dst, src, bytes, lane);
         else if (CAST == 0)
           warp_copy_simt(dst, src, bytes, lane);
@@ -460,37 +438,20 @@ __device__ __forceinline__ void ring_consumer(const RingSmem& sm, int ndst_rt, c
         ptx::mbar_arrive(sm.empty0 + 8 * slot);
         ptx::bulk_commit();  // always one group per item (possibly empty) so the wait_group counts hold
       }
-    } else if (CAST == 0 && variant == 0) {
+    } else if (CAST == 0 && !multimem) {
       if (lane == 0) {
 #pragma unroll
         for (int d = 0; d < kMaxDst; ++d)
-          if (d < ndst) {
-            if (cache_hint & 2)
-              ptx::bulk_s2g_hint(reinterpret_cast<void*>(c.dst[d]), in, bytes, policy);
-            else
-              ptx::bulk_s2g(reinterpret_cast<void*>(c.dst[d]), in, bytes);
-          }
+          if (d < ndst) ptx::bulk_s2g(reinterpret_cast<void*>(c.dst[d]), in, bytes);
         ptx::bulk_commit();
         deferred |= 1u << (q & 31);
       }
-    } else if (CAST == 0) {  // variants 1, 2, 3, 4: the slot is released synchronously
-      if (variant == 1) {
-        for (int d = 0; d < ndst; ++d) warp_store_from_smem(reinterpret_cast<uint8_t*>(c.dst[d]), in, bytes, lane);
-      } else if (variant == 4) {
-        warp_store_from_smem_mc(reinterpret_cast<uint8_t*>(c.dst[0]), in, bytes, lane);
-      } else if (variant == 3) {  // stores only: whatever is in the slot
-        if (lane == 0) {
-#pragma unroll
-          for (int d = 0; d < kMaxDst; ++d)
-            if (d < ndst) ptx::bulk_s2g(reinterpret_cast<void*>(c.dst[d]), in, bytes);
-          ptx::bulk_commit();
-          ptx::bulk_wait_read<0>();
-        }
-      }
+    } else if (CAST == 0) {  // multimem: the warp's stores have read the slot, so it is released right away
+      warp_store_from_smem_mc(reinterpret_cast<uint8_t*>(c.dst[0]), in, bytes, lane);
       __syncwarp();
       if (lane == 0) {
         ptx::mbar_arrive(sm.empty0 + 8 * slot);
-        if (variant != 3) ptx::bulk_commit();
+        ptx::bulk_commit();
       }
     } else {
       const uint32_t dst_bytes = CAST == 1 ? bytes * 2 : bytes / 2;

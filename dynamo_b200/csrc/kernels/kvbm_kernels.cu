@@ -9,7 +9,6 @@
 #include <atomic>
 #include <mutex>
 #include <cstdio>
-#include <cstdlib>
 #include <vector>
 
 namespace kvbm {
@@ -196,9 +195,10 @@ static void sched_release(int dev, int slot, cudaStream_t stream)
 // ------------------------------------------------------------------------------------------------
 constexpr uint32_t kPairChunk = 32768;
 constexpr uint32_t kPairSmall = 4096;
+constexpr int kPairUnroll = 4;
+constexpr int kPairThreads = 256;
 
-template <int U>
-__global__ void __launch_bounds__(256)
+__global__ void __launch_bounds__(kPairThreads)
 kvbm_pair_copy_kernel(void* const* __restrict__ src_ptrs, void* const* __restrict__ dst_ptrs, size_t copy_size,
                       uint32_t chunks_per_pair, uint64_t num_pairs)
 {
@@ -206,7 +206,8 @@ kvbm_pair_copy_kernel(void* const* __restrict__ src_ptrs, void* const* __restric
   if (copy_size <= kPairSmall) {  // warp per pair
     const uint64_t pair = bid * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (pair >= num_pairs) return;
-    group_copy_simt<U>(static_cast<uint8_t*>(dst_ptrs[pair]), static_cast<const uint8_t*>(src_ptrs[pair]), copy_size, threadIdx.x & 31, 32);
+    group_copy_simt<kPairUnroll>(static_cast<uint8_t*>(dst_ptrs[pair]), static_cast<const uint8_t*>(src_ptrs[pair]), copy_size,
+                                 threadIdx.x & 31, 32);
     return;
   }
   const uint64_t pair = bid / chunks_per_pair;
@@ -215,8 +216,8 @@ kvbm_pair_copy_kernel(void* const* __restrict__ src_ptrs, void* const* __restric
   const size_t off = static_cast<size_t>(chunk) * kPairChunk;
   const size_t left = copy_size - off;
   // chunk boundaries are multiples of 32 KiB, so the alignment class of (src, dst) is the same for every chunk
-  group_copy_simt<U>(static_cast<uint8_t*>(dst_ptrs[pair]) + off, static_cast<const uint8_t*>(src_ptrs[pair]) + off,
-                     left < kPairChunk ? left : kPairChunk, threadIdx.x, blockDim.x);
+  group_copy_simt<kPairUnroll>(static_cast<uint8_t*>(dst_ptrs[pair]) + off, static_cast<const uint8_t*>(src_ptrs[pair]) + off,
+                               left < kPairChunk ? left : kPairChunk, threadIdx.x, blockDim.x);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -343,14 +344,13 @@ __device__ __forceinline__ StreamSync make_sync(const PagedSyncArgs& s, const Pa
 template <int CAST, bool FAST>
 __global__ void __launch_bounds__(512, 1)
 kvbm_paged_copy_kernel(const __grid_constant__ PagedGen gen, const __grid_constant__ PagedSyncArgs sync,
-                       uint32_t total, int S, int P, int batch, int static_schedule, uint32_t out_tile, int allow_tma, int cache_hint,
-                       int variant)
+                       uint32_t total, int S, int P, int batch, int static_schedule, uint32_t out_tile, int allow_tma, int multimem)
 {
   extern __shared__ __align__(128) uint8_t smem[];
   const int R = blockDim.x >> 6;
   const int ring_ndst = gen.a.replicate ? gen.a.ndst : 1;
   const StreamSync ss = make_sync(sync, gen.a, total, R);
-  RingParams rp{S, P, batch, gen.a.tile, out_tile, allow_tma != 0, static_schedule != 0, cache_hint, CAST == KVBM_CAST_NONE ? variant : 0};
+  RingParams rp{S, P, batch, gen.a.tile, out_tile, allow_tma != 0, static_schedule != 0, CAST == KVBM_CAST_NONE && multimem != 0};
   run_rings<CAST, FAST>(smem, gen, total, ring_ndst, rp, ss);
 }
 
@@ -652,10 +652,7 @@ static cudaError_t preload_kernels()
   cudaError_t e;
 #define KVBM_PRELOAD(k) \
   if ((e = cudaFuncGetAttributes(&attr, k)) != cudaSuccess) return e;
-  KVBM_PRELOAD(kvbm_pair_copy_kernel<8>)
-  KVBM_PRELOAD(kvbm_pair_copy_kernel<4>)
-  KVBM_PRELOAD(kvbm_pair_copy_kernel<2>)
-  KVBM_PRELOAD(kvbm_pair_copy_kernel<1>)
+  KVBM_PRELOAD(kvbm_pair_copy_kernel)
   KVBM_PRELOAD((kvbm_paged_copy_kernel<KVBM_CAST_NONE, false>))
   KVBM_PRELOAD((kvbm_paged_copy_kernel<KVBM_CAST_FP8E4M3_TO_BF16, false>))
   KVBM_PRELOAD((kvbm_paged_copy_kernel<KVBM_CAST_BF16_TO_FP8E4M3, false>))
@@ -732,7 +729,8 @@ kvbm_kernels_launch_vectorized_copy(void** src_ptrs, void** dst_ptrs, size_t cop
   uint64_t ctas;
   uint32_t chunks_per_pair = 1;
   if (copy_size_bytes <= kPairSmall) {
-    ctas = (pairs + 7) / 8;  // 8 warps per CTA, one pair each
+    constexpr uint64_t warps = kPairThreads / 32;  // one pair per warp
+    ctas = (pairs + warps - 1) / warps;
   } else {
     const uint64_t cpp = (copy_size_bytes + kPairChunk - 1) / kPairChunk;
     if (cpp >= (1ull << 32)) return cudaErrorInvalidValue;
@@ -742,17 +740,8 @@ kvbm_kernels_launch_vectorized_copy(void** src_ptrs, void** dst_ptrs, size_t cop
   const uint64_t gx = std::min<uint64_t>(ctas, 1ull << 30);
   const uint64_t gy = (ctas + gx - 1) / gx;
   if (gy > 65535) return cudaErrorInvalidValue;
-  // tuning knobs for experiments (benchmarks/kvbench.py): loads in flight per thread and CTA width
-  static const int k1_unroll = [] { const char* e = std::getenv("KVBM_K1_UNROLL"); return e ? std::atoi(e) : 4; }();
-  static const int k1_threads = [] { const char* e = std::getenv("KVBM_K1_THREADS"); const int t = e ? std::atoi(e) : 256; return t >= 32 && t <= 256 && t % 32 == 0 ? t : 256; }();
-  if (copy_size_bytes <= kPairSmall) ctas = (pairs + (k1_threads / 32) - 1) / (k1_threads / 32);
-  const dim3 grid(static_cast<unsigned>(std::min<uint64_t>(ctas, 1ull << 30)), static_cast<unsigned>((ctas + std::min<uint64_t>(ctas, 1ull << 30) - 1) / std::min<uint64_t>(ctas, 1ull << 30)));
-  switch (k1_unroll) {
-    case 1: kvbm_pair_copy_kernel<1><<<grid, k1_threads, 0, stream>>>(src_ptrs, dst_ptrs, copy_size_bytes, chunks_per_pair, pairs); break;
-    case 2: kvbm_pair_copy_kernel<2><<<grid, k1_threads, 0, stream>>>(src_ptrs, dst_ptrs, copy_size_bytes, chunks_per_pair, pairs); break;
-    case 8: kvbm_pair_copy_kernel<8><<<grid, k1_threads, 0, stream>>>(src_ptrs, dst_ptrs, copy_size_bytes, chunks_per_pair, pairs); break;
-    default: kvbm_pair_copy_kernel<4><<<grid, k1_threads, 0, stream>>>(src_ptrs, dst_ptrs, copy_size_bytes, chunks_per_pair, pairs); break;
-  }
+  const dim3 grid(static_cast<unsigned>(gx), static_cast<unsigned>(gy));
+  kvbm_pair_copy_kernel<<<grid, kPairThreads, 0, stream>>>(src_ptrs, dst_ptrs, copy_size_bytes, chunks_per_pair, pairs);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   return cudaGetLastError();  // :570
 }
@@ -963,6 +952,7 @@ paged_copy_impl(const kvbm_paged_layout* src, const kvbm_paged_dst* dsts, int nu
 
   kvbm_paged_copy_opts o{};
   if (opts) o = *opts;
+  if (o.reserved0 != 0 || o.reserved1 != 0) return cudaErrorInvalidValue;
 
   // NVLS: dsts[0] is addressed through a multicast mapping and carries the payload for every bound device; the
   // other entries only name the flags of the remaining receivers.
@@ -1044,7 +1034,7 @@ paged_copy_impl(const kvbm_paged_layout* src, const kvbm_paged_dst* dsts, int nu
     cudaError_t err = set_smem(kern, rc.smem);
     if (err == cudaSuccess) {
       kern<<<grid, rc.rings * 64, rc.smem, stream>>>(gen, sync, total32, rc.stages, rc.pending, rc.batch, o.static_schedule,
-                                                     rc.out_tile, allow_tma, o.cache_hint, mc ? (o.multicast == 2 ? 0 : 4) : o.variant);
+                                                     rc.out_tile, allow_tma, mc && o.multicast != 2);
       g_launches.fetch_add(1, std::memory_order_relaxed);
       err = cudaGetLastError();
     }
@@ -1054,7 +1044,7 @@ paged_copy_impl(const kvbm_paged_layout* src, const kvbm_paged_dst* dsts, int nu
   // the plain hot path gets the kernel with the generality folded away at compile time (copy_engine.cuh, FAST)
   bool any_layer_flags = false;
   for (int d = 0; d < num_dsts; ++d) any_layer_flags = any_layer_flags || dsts[d].layer_done_flags != nullptr;
-  const bool fast = !mc && o.variant == 0 && o.cache_hint == 0 && allow_tma && !o.layer_ready_flags && !any_layer_flags &&
+  const bool fast = !mc && allow_tma && !o.layer_ready_flags && !any_layer_flags &&
                     (gen.a.replicate ? data_dsts : 1) == 1;
   switch (cast_mode) {
     case KVBM_CAST_NONE:

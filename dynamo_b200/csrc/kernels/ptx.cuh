@@ -64,26 +64,11 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src_gmem
       "l"(src_gmem), "r"(bytes), "r"(bar)
       : "memory");
 }
-__device__ __forceinline__ void bulk_g2s_hint(uint32_t dst_smem, const void* src_gmem,
-                                              uint32_t bytes, uint32_t bar, uint64_t policy)
-{
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, "
-      "[%3], %4;" ::"r"(dst_smem),
-      "l"(src_gmem), "r"(bytes), "r"(bar), "l"(policy)
-      : "memory");
-}
 // shared -> global (local HBM or an NVLink peer mapping), tracked by bulk async-groups.
 __device__ __forceinline__ void bulk_s2g(void* dst_gmem, uint32_t src_smem, uint32_t bytes)
 {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst_gmem),
                "r"(src_smem), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_s2g_hint(void* dst_gmem, uint32_t src_smem, uint32_t bytes, uint64_t policy)
-{
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(dst_gmem),
-               "r"(src_smem), "r"(bytes), "l"(policy)
                : "memory");
 }
 __device__ __forceinline__ void bulk_commit()
@@ -122,13 +107,6 @@ __device__ __forceinline__ void bulk_wait()
 {
   asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
 }
-__device__ __forceinline__ uint64_t policy_evict_first()
-{
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-
 // generic-proxy writes to smem -> visible to the async proxy (before a bulk store reads them)
 __device__ __forceinline__ void fence_proxy_async_smem()
 {

@@ -112,8 +112,8 @@ class PagedCopyOpts(C.Structure):
         ("completion_flag", C.c_void_p),
         ("completion_value", C.c_uint32),
         ("stores_in_flight", C.c_int),
-        ("cache_hint", C.c_int),
-        ("variant", C.c_int),
+        ("reserved0", C.c_int),
+        ("reserved1", C.c_int),
         ("gate_timeout_ms", C.c_int),
         ("multicast", C.c_int),
         ("gate_mode", C.c_int),

@@ -137,11 +137,10 @@ typedef struct kvbm_paged_copy_opts {
                                      completion_value once EVERY destination has landed: lets the host
                                      observe completion without cudaEventQuery polling */
   uint32_t completion_value;
-  int stores_in_flight;           /* 0 = default (stages/2): slots that may still be draining to the destination;
+  int stores_in_flight;           /* 0 = default (max(1, stages/3)): slots that may still be draining to the destination;
                                      stages - stores_in_flight loads are kept in flight ahead */
-  int cache_hint;                 /* bit0: L2 evict_first on source reads, bit1: on destination writes */
-  int variant;                    /* 0 = TMA load + TMA store (default); 1 = TMA load + SIMT store from smem;
-                                     2 / 3 = loads-only / stores-only DIAGNOSTICS (do not copy correctly) */
+  int reserved0;                  /* must be 0 (keeps the offsets of the fields below); non-zero -> cudaErrorInvalidValue */
+  int reserved1;                  /* must be 0 (keeps the offsets of the fields below); non-zero -> cudaErrorInvalidValue */
   int gate_timeout_ms;            /* gated transfers: a layer_ready wait longer than this aborts the launch (completion word
                                      becomes 0xFFFFFFFF, done flags are not written) instead of hanging the GPU; 0 = 10 s */
   int multicast;                  /* NVLS: non-zero = dsts[0].layout.layer_base[] hold NVLink MULTICAST addresses (a mapping of a

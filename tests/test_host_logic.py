@@ -77,6 +77,18 @@ def test_library_loads_without_gpu_and_reports_real_build():
     assert K.memcpy_batch(None, None, 64, 3, K.MemcpyBatchMode.FallbackOnly, 0) == K.CUDA_ERROR_INVALID_VALUE
 
 
+def test_paged_copy_rejects_nonzero_reserved_option_fields():
+    """kvbm_paged_copy_opts.reserved0 / reserved1 must be 0.  The slots once selected L2 cache hints and diagnostic ring
+    variants that did not copy; a caller that still sets them gets cudaErrorInvalidValue, before any CUDA call, instead of
+    a transfer.  The arguments are otherwise well-formed; their addresses are never dereferenced."""
+    region, nl, no, nb = 4096, 2, 2, 8
+    layout = lambda base: K.PagedLayout(base, no * region, region, region, nl, no, nb)
+    dst = K.PagedDst(layout(0x200000), 0x300000, 0x400000, 0, 0)
+    for field, value in (("reserved0", 1), ("reserved1", 2)):
+        opts = K.PagedCopyOpts(**{field: value})
+        assert K.paged_copy(layout(0x100000), [dst], 4, 0, nl, K.CastMode.NONE, opts) == K.CUDA_ERROR_INVALID_VALUE, field
+
+
 def test_product_never_imports_the_oracle():
     pkg = os.path.join(ROOT, "dynamo_b200")
     for base, _, files in os.walk(pkg):
